@@ -2,6 +2,7 @@
 """Benchmark of the HippoRAG retrieval hot path on B200 (contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C1|C2|C3|C5] [--impl reference]
+                    [--dump-outputs DIR]
 
 A *step* = one batch of ``--queries`` queries through the whole path
 (stage A: query x fact similarity + top-5 -> identity recognition-memory filter -> stage B:
@@ -313,6 +314,24 @@ def load_engine(eng, wl, args_obj=None):
         eng.load_embeddings(wl.fe, wl.pe)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ids, scores):
+    """What ``retrieve_resident`` hands its caller: top-k passage ids (as float64, exact for int32) and scores
+    (float32), one row per query.  Batches too large for DUMP_BYTES keep a fixed seeded sample of rows, listed in
+    ``rows.npy``, so two builds run with the same arguments can be compared row for row."""
+    row_bytes = ids.shape[1] * 8 + scores.shape[1] * 4 + 8
+    rows = np.arange(ids.shape[0])
+    if rows.size * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(rows.size, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "topk_ids.npy"), ids[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "topk_scores.npy"), scores[rows].astype(np.float32))
+    log(f"[bench] outputs of the last timed step ({rows.size} of {ids.shape[0]} queries) written to {out_dir}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -332,8 +351,12 @@ def main():
     ap.add_argument("--cpu-best-effort-sample", type=int, default=128, help="queries in the best-effort CPU leg (0 = skip)")
     ap.add_argument("--ref-queries", type=int, default=4, help="queries per step of --impl reference")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the top-k ids and scores of the last timed step to DIR/*.npy (rank 0's batch)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     # one JSON line on stdout: NCCL prints its version banner (levels VERSION and WARN) and its INFO log there
     if os.environ.get("NCCL_DEBUG", "").upper() in ("VERSION", "WARN"):
@@ -450,6 +473,8 @@ def main():
                    "d2h_bytes_per_step": int(st2["d2h_bytes"] // args.steps), "ms_per_step": ms_e2e / args.steps}
         res = dict(ms_total=ms_total, st=st, clocks=clocks, e2e=e2e, out_ids=out_ids[:max(args.cpu_sample, 8)].cpu().numpy(),
                    h_qf=h_qf_np, h_qp=h_qp_np)
+        if args.dump_outputs and mode == head_mode:
+            res["dump"] = (out_ids.cpu().numpy(), out_scores.cpu().numpy())   # still the last timed step's results
         eng.close()
         del eng
         torch.cuda.empty_cache()
@@ -475,6 +500,8 @@ def main():
         return
 
     peak, peak_src = measured_peaks()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *main_res["dump"])
 
     def roofline_of(res, mode):
         st = res["st"]

@@ -2,6 +2,8 @@
 ``hipporag.utils.misc_utils`` the drop-in imports), for boxes where /root/reference is absent.
 Only what ``hipporag_b200.accelerate`` touches is modelled."""
 import hashlib
+import json
+import os
 import sys
 import types
 from dataclasses import dataclass
@@ -180,3 +182,66 @@ class FakeRag:
 
     def delete(self, docs):
         self.ready_to_retrieve = False
+
+
+class RecordedRag(FakeRag):
+    """The reference's own ``HippoRAG`` object as its ``index()`` left it, rebuilt from the recording
+    ``tests/golden/reference_rag150.npz`` (``tests/golden/make_reference_rag.py``): graph, stores,
+    ``ent_node_to_chunk_ids`` and config as recorded; embeddings regenerated from the stored texts by the
+    md5-seeded mock embedder the recording was made with.  ``prepare_retrieval_objects``,
+    ``get_query_embeddings`` and the IRCoT prompt follow HippoRAG.py:1287-1389, :1391-1425 and qa_utils.py:31-50."""
+
+    def __init__(self, g, working_dir):
+        from hipporag.utils.misc_utils import compute_mdhash_id
+        from oracle.ref_harness import MockEmbeddingModel, identity_filter
+        self.global_config = types.SimpleNamespace(**json.loads(str(g["config"])))
+        self.working_dir = working_dir
+        self.passage_texts, self.fact_texts = g["passage_texts"].tolist(), g["fact_texts"].tolist()
+        ent_texts = g["entity_texts"].tolist()
+        self.passage_node_keys = [compute_mdhash_id(t, prefix="chunk-") for t in self.passage_texts]
+        self.fact_node_keys = [compute_mdhash_id(t, prefix="fact-") for t in self.fact_texts]
+        self.entity_keys = [compute_mdhash_id(t, prefix="entity-") for t in ent_texts]
+        names = [(self.entity_keys + self.passage_node_keys)[i] for i in g["vertex_key"]]
+        graph = Graph(directed=False)
+        graph.add_vertices(len(names), attributes={"name": names})
+        graph.add_edges(list(zip(g["edge_src"].tolist(), g["edge_dst"].tolist())),
+                        attributes={"weight": g["edge_w"].tolist()})
+        self.graph = graph
+        self.fact_embedding_store = _Store(self.fact_node_keys, self.fact_texts)
+        self.chunk_embedding_store = _Store(self.passage_node_keys, self.passage_texts)
+        self.ent_node_to_chunk_ids = {self.entity_keys[i]: set(range(int(c)))
+                                      for i, c in zip(g["chunk_count_entity"], g["chunk_counts"])}
+        self.embedding_model = MockEmbeddingModel(int(g["dim"]))
+        self._instruction = {"triple": str(g["query_instruction_fact"]), "passage": str(g["query_instruction_passage"])}
+        self.entity_embedding_store = _Store(self.entity_keys, ent_texts)
+        self.entity_embedding_store.emb = self.embedding_model.batch_encode(ent_texts)
+        self.entity_embedding_store.index = {k: i for i, k in enumerate(self.entity_keys)}
+        self.node_to_node_stats = {}
+        self.prompt_template_manager = types.SimpleNamespace(
+            is_template_name_valid=lambda name: True,
+            render=lambda name, prompt_user: [{"role": "user", "content": prompt_user}])
+        self.chunk_metadata = {}
+        self.ready_to_retrieve = False
+        self.ppr_time = self.rerank_time = self.all_retrieval_time = 0.0
+        self.rerank_filter = identity_filter
+
+    def prepare_retrieval_objects(self):
+        self.query_to_embedding = {"triple": {}, "passage": {}}
+        self.node_name_to_vertex_idx = {n: i for i, n in enumerate(self.graph.vs["name"])}
+        self.passage_node_idxs = [self.node_name_to_vertex_idx[k] for k in self.passage_node_keys]
+        self.passage_embeddings = self.embedding_model.batch_encode(self.passage_texts)
+        self.fact_embeddings = self.embedding_model.batch_encode(self.fact_texts)
+        self.ready_to_retrieve = True
+
+    def get_query_embeddings(self, queries):
+        new = [q for q in queries if q not in self.query_to_embedding["triple"]
+               or q not in self.query_to_embedding["passage"]]
+        for kind in ("triple", "passage") if new else ():
+            emb = self.embedding_model.batch_encode(new, instruction=self._instruction[kind])
+            self.query_to_embedding[kind].update(zip(new, emb))
+
+
+def load_recorded_rag(working_dir):
+    """-> (the recording's arrays, a RecordedRag built from them that keeps its index cache in working_dir)."""
+    g = dict(np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_rag150.npz")))
+    return g, RecordedRag(g, working_dir)

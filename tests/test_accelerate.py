@@ -1,7 +1,7 @@
-"""The drop-in (hipporag_b200.accelerate): host glue against the reference's own object (CPU,
-oracle-backed engine double) and the GPU path through a duck-typed HippoRAG (GPU box)."""
+"""The drop-in (hipporag_b200.accelerate): host glue against the reference's own object, replayed from a
+recording (CPU, oracle-backed engine double), and the GPU path through a duck-typed HippoRAG (GPU box)."""
+import json
 import os
-import tempfile
 
 import numpy as np
 import pytest
@@ -62,48 +62,57 @@ class OracleEngine:
         return ids, sc
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout")
-def test_accelerate_glue_against_reference_object():
-    from oracle import ref_harness as H
+class FakeQALLM:
+    """IRCoT reasoning double: the thought depends on the question and on how many thoughts came before."""
+
+    def infer(self, messages):
+        text = messages[-1]["content"] if isinstance(messages[-1], dict) else str(messages[-1])
+        q = text.rsplit("Question:", 1)[-1]
+        n_prev = q.count("thought-")
+        tag = "thought-%d about %s" % (n_prev, q.split("\n")[0].strip()[:40])
+        return [tag + (" So the answer is: x" if n_prev >= 1 and len(q) % 2 == 0 else "")]
+
+
+def test_accelerate_glue_against_reference_object(tmp_path):
+    """The reference's own HippoRAG object, replayed from tests/golden/reference_rag150.npz (state after its index()
+    and what its own retrieve / retrieve_ircot returned; see tests/golden/make_reference_rag.py)."""
+    from tests import fake_hipporag
+    fake_hipporag.install_stub_package()
     import hipporag_b200
-    rag = H.build_reference_rag(tempfile.mkdtemp(prefix="hrag_acc_"), 150, 64)
-    questions = H.musique_questions(12)
-    ref = rag.retrieve(questions, num_to_retrieve=20)
+    from hipporag.utils.misc_utils import QuerySolution
+    g, rag = fake_hipporag.load_recorded_rag(str(tmp_path))
+    questions = g["questions"].tolist()
+    ref_docs = [[rag.passage_texts[i] for i in row] for row in g["ref_doc_ids"]]
+    ref_seeds = json.loads(str(g["ref_graph_seeds"]))
     hipporag_b200.accelerate(rag, engine=OracleEngine())
     rag.ready_to_retrieve = False
     acc = rag.retrieve(questions, num_to_retrieve=20)
-    assert len(acc) == len(ref)
+    assert len(acc) == len(ref_docs)
     same = 0
-    for a, r in zip(acc, ref):
-        assert a.question == r.question and len(a.docs) == len(r.docs) == 20
-        assert type(a) is type(r)
-        overlap = len(set(a.docs) & set(r.docs)) / 20
+    for a, q, r_docs, r_scores, r_seeds in zip(acc, questions, ref_docs, g["ref_doc_scores"], ref_seeds):
+        assert a.question == q and len(a.docs) == len(r_docs) == 20
+        assert type(a) is QuerySolution
+        overlap = len(set(a.docs) & set(r_docs)) / 20
         assert overlap >= 0.8
-        assert [tuple(f) for f in a.graph_seeds] == [tuple(f) for f in r.graph_seeds]
-        if a.docs == r.docs and np.allclose(a.doc_scores, r.doc_scores, rtol=1e-5):
+        assert [tuple(f) for f in a.graph_seeds] == [tuple(f) for f in r_seeds]
+        if a.docs == r_docs and np.allclose(a.doc_scores, r_scores, rtol=1e-5):
             same += 1
-    assert same >= len(ref) // 2          # the rest differ only by the reference's set-order tie-break
+    assert same >= len(ref_docs) // 2          # the rest differ only by the reference's set-order tie-break
     assert rag.all_retrieval_time > 0 and rag.ppr_time > 0
     # the thread-pooled filter gives the same answers as the serial one
     hipporag_b200.accelerate(rag, engine=OracleEngine(), filter_workers=4)
     rag.ready_to_retrieve = False
     par = rag.retrieve(questions, num_to_retrieve=20)
     assert [p.docs for p in par] == [a.docs for a in acc]
-    # IRCoT: the batched, step-synchronous drop-in must equal the reference's serial loop
-    class FakeQALLM:
-        def infer(self, messages):
-            text = messages[-1]["content"] if isinstance(messages[-1], dict) else str(messages[-1])
-            q = text.rsplit("Question:", 1)[-1]
-            n_prev = q.count("thought-")
-            tag = "thought-%d about %s" % (n_prev, q.split("\n")[0].strip()[:40])
-            return [tag + (" So the answer is: x" if n_prev >= 1 and len(q) % 2 == 0 else "")]
+    # IRCoT: the batched, step-synchronous drop-in must equal the reference's serial loop (HippoRAG.py:509)
     rag.qa_llm = FakeQALLM()
-    serial_ircot = type(rag).retrieve_ircot                    # the reference's own method (HippoRAG.py:509)
-    want = serial_ircot(rag, questions[:6], max_qa_steps=3, num_to_retrieve=10)
     got = rag.retrieve_ircot(questions[:6], max_qa_steps=3, num_to_retrieve=10)
-    for a, b in zip(got, want):
-        assert a.docs == b.docs and a.thoughts == b.thoughts
-        np.testing.assert_allclose(a.doc_scores, b.doc_scores)
+    want = zip(json.loads(str(g["ircot_doc_ids"])), json.loads(str(g["ircot_doc_scores"])),
+               json.loads(str(g["ircot_thoughts"])))
+    assert len(got) == 6
+    for a, (b_ids, b_scores, b_thoughts) in zip(got, want):
+        assert a.docs == [rag.passage_texts[i] for i in b_ids] and a.thoughts == b_thoughts
+        np.testing.assert_allclose(a.doc_scores, b_scores)
     # the binary cache (8(f)-3): written next to graph.pickle on the first prepare, reused while the index is unchanged
     import sys as _sys
     from hipporag_b200 import cache as cache_mod
@@ -135,12 +144,12 @@ def test_accelerate_glue_against_reference_object():
     orig_filter = rag.rerank_filter
     rag.rerank_filter = lambda q, c, i, len_after_rerank=None: (seen.append(len(c)) or (i[:len_after_rerank], c[:len_after_rerank], {}))
     rag.global_config.linking_top_k = 10
-    ref10 = type(rag).retrieve(rag, questions[:4], num_to_retrieve=10)      # the reference's own method
+    ref10 = json.loads(str(g["ref10_graph_seeds"]))                          # the reference's own retrieve
     seen.clear()
     acc10 = rag.retrieve(questions[:4], num_to_retrieve=10)
-    assert seen == [10, 10, 10, 10]
+    assert seen == [10, 10, 10, 10] and len(ref10) == 4
     for a, r in zip(acc10, ref10):
-        assert [tuple(f) for f in a.graph_seeds] == [tuple(f) for f in r.graph_seeds] and len(a.graph_seeds) == 10
+        assert [tuple(f) for f in a.graph_seeds] == [tuple(f) for f in r] and len(a.graph_seeds) == 10
     rag.global_config.linking_top_k = 40
     with pytest.raises(ValueError, match="linking_top_k"):
         rag.retrieve(questions[:2], num_to_retrieve=5)
@@ -148,7 +157,7 @@ def test_accelerate_glue_against_reference_object():
     rag.rerank_filter = orig_filter
     # add_synonymy_edges is wrapped: the KNN it calls is swapped for the engine's for the duration of the call only
     import sys
-    ref_mod = sys.modules[type(rag).__module__]              # hipporag.HippoRAG, the module (the package re-exports the class)
+    ref_mod = sys.modules[type(rag).__module__]              # the module whose retrieve_knn add_synonymy_edges calls
     from hipporag_b200 import knn as knn_mod
     calls = {}
 

@@ -4,7 +4,6 @@ import json
 import os
 import subprocess
 import sys
-import tempfile
 
 import numpy as np
 import pytest
@@ -58,20 +57,43 @@ def test_roofline_byte_model():
     assert 3000 < peak < 9000 and ("measured" in src or "fallback" in src)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout")
-def test_dropin_table_extraction_matches_the_harness():
+def test_dropin_table_extraction_matches_the_harness(tmp_path):
     """accelerate.extract_tables (product) and oracle.ref_harness.extract_tables (test infrastructure) are
-    written independently from the same reference lines; on the reference's own object they must agree."""
-    from oracle import ref_harness as H
+    written independently from the same reference lines; on the reference's own object (replayed from
+    tests/golden/reference_rag150.npz, which holds what the harness extracted from it) they must agree."""
+    from tests import fake_hipporag
+    fake_hipporag.install_stub_package()
     from hipporag_b200.accelerate import extract_tables
-    rag = H.build_reference_rag(tempfile.mkdtemp(prefix="hrag_tb_"), 120, 32)
-    want = H.extract_tables(rag)
+    g, rag = fake_hipporag.load_recorded_rag(str(tmp_path))
+    rag.prepare_retrieval_objects()
+    want = {k: g[k] for k in ("edge_src", "edge_dst", "edge_w")}
+    want.update({k: g["harness_" + k] for k in ("n_nodes", "passage_vid", "fact_subj_vid", "fact_obj_vid",
+                                                "ent_chunk_count")})
     got = extract_tables(rag)
     for k in ("n_nodes", "edge_src", "edge_dst", "edge_w", "passage_vid", "fact_subj_vid", "fact_obj_vid",
               "ent_chunk_count"):
         assert np.array_equal(np.asarray(got[k]), np.asarray(want[k])), k
-    assert [str(f) for f in got["facts"]] == want["fact_texts"]
+    assert [str(f) for f in got["facts"]] == g["fact_texts"].tolist()
     assert (got["fact_subj_vid"] >= 0).all() and (got["ent_chunk_count"][got["passage_vid"]] == 0).all()
+
+
+def test_bench_dump_outputs_fixed_sample_within_budget(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(1)
+    ids = rng.integers(0, 1 << 30, (300, 200)).astype(np.int32)
+    scores = rng.random((300, 200)).astype(np.float32)
+    bench.dump_outputs(str(tmp_path / "all"), ids, scores)
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "topk_ids.npy"), ids)
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "topk_scores.npy"), scores)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * (200 * 12 + 8))      # room for 100 of the 300 rows
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ids, scores)
+    rows = np.load(tmp_path / "a" / "rows.npy").astype(np.int64)
+    assert rows.size == 100 and np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    got = np.load(tmp_path / "a" / "topk_ids.npy")
+    assert got.dtype == np.float64 and np.array_equal(got, ids[rows])
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES + 3 * 128
 
 
 def test_reference_arm_prints_one_contract_line():
