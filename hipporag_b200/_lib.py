@@ -64,7 +64,7 @@ SIGNATURES = {
     "hrag_topk_similarity": (C.c_int, [_p, C.c_int, _i32, _p, _i32, _p, _p]),
     "hrag_knn_threshold": (C.c_int, [_p, C.c_int, _i32, _p, _f32, _i32, _p, _p, _p]),
     "hrag_bench_sweep": (C.c_int, [_p, _i32, _i32, _i32, C.POINTER(_f32)]),
-    "hrag_set_tuning": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "hrag_set_tuning": (C.c_int, [_p, C.c_int]),
     "hrag_stream": (_p, [_p]),
     "hrag_get_stats": (C.c_int, [_p, C.POINTER(Stats)]),
     "hrag_reset_stats": (C.c_int, [_p]),

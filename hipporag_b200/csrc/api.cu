@@ -146,9 +146,6 @@ struct hrag_handle {
     Buf H0b, mixed_aux1, prep_scratch;
     Buf slot_map[2], slot_vid[2], Vc[2], R16[2], rho;
     bool slot_maps_valid = false;
-    alignas(128) unsigned char xmap[5][128];   // CUtensorMap of H[0..3], H0b for the TMA-gather sweep (K1t)
-    bool xmaps_valid = false;
-    int use_tma = -1;                          // HRAG_MIXED_TMA=1 routes plain fp16 sweeps through k_sweep_h_tma
     // CUDA graphs of the mixed solve, one per (buffer set, sweep plan); `graph_generation` changes whenever anything a
     // captured launch depends on does (graph / tables reload, state reallocation, tuning switches)
     struct SolveGraph {
@@ -162,7 +159,6 @@ struct hrag_handle {
     };
     std::vector<SolveGraph> solve_graphs;
     int64_t graph_generation = 0;
-    int use_graphs = -1;                       // HRAG_PPR_GRAPHS=0 disables
     int k5_debug = 0;                          // profiling switches of the fused exchange (SweepSync::debug)
     unsigned int* d_done_ctr = nullptr;
     // one allocation [H0 | H1 | H2 | H3 | H0b | flags] so a single IPC handle exposes every buffer a peer
@@ -315,14 +311,7 @@ int ensure_state_mixed(hrag_t* h) {
             HRAG_CUDA(cudaMalloc(&h->d_done_ctr, sizeof(unsigned int)));
             HRAG_CUDA(cudaMemset(h->d_done_ctr, 0, sizeof(unsigned int)));
         }
-        h->xmaps_valid = false;
         h->graph_generation += 1;
-    }
-    if (h->use_tma < 0) { const char* e = getenv("HRAG_MIXED_TMA"); h->use_tma = e ? atoi(e) : 0; }
-    if (h->use_tma && !h->xmaps_valid) {
-        hrag::Buf* views[5] = {&h->H[0], &h->H[1], &h->H[2], &h->H[3], &h->H0b};
-        for (int i = 0; i < 5; ++i) HRAG_TRY(tma_state_map(views[i]->p, (int64_t)rows, h->xmap[i]));
-        h->xmaps_valid = true;
     }
     HRAG_TRY(h->partials.ensure((size_t)std::max(mixed_partial_rows(h->g), 1024) * 32 * sizeof(float)));
     HRAG_TRY(h->sums.ensure(192 * sizeof(double)));      // sums of x0, of d, of |r|, and of v (two sets)
@@ -427,13 +416,6 @@ int p2p_signal(hrag_t* h) {
 int mixed_sweep_x(hrag_t* h, int mode, const void* x, const int* slot_map, const void* rhs, const float* v32,
                   const float* scale, const void* prev, void* y, float alpha, float w, float t, float* part,
                   int* n_part) {
-    if (h->use_tma == 1 && mode == 0 && part == nullptr && !h->p2p && h->g.n_long == 0 && h->xmaps_valid) {
-        // K1t: gathered rows through TMA gather4 (x is one of the five slab buffers)
-        const int xi = (int)((static_cast<const char*>(x) - static_cast<const char*>(h->slab)) / (ptrdiff_t)h->slab_hb);
-        HRAG_CHECK(xi >= 0 && xi < 5, "internal: x is not a slab buffer");
-        HRAG_TRY(mixed_sweep_tma(h->g, h->xmap[xi], slot_map, rhs, prev, y, alpha, w, peers_for(h, y), h->stream));
-        return exchange_rows_bytes(h, y, 32 * 2);
-    }
     HRAG_TRY(mixed_sweep(h->g, mode, x, slot_map, rhs, v32, scale, prev, y, alpha, w, t, part, n_part, peers_for(h, y),
                          sync_for_sweep(h), h->stream));
     if (!h->p2p) HRAG_TRY(exchange_rows_bytes(h, y, 32 * 2));
@@ -553,12 +535,11 @@ int dev_ppr_mixed_body(hrag_t* h, const SweepPlan& plan, float alpha, const int*
 // The solve of one sub-batch is ~20 launches whose arguments depend only on the buffer set and the sweep plan, so on a
 // single GPU it is captured once per (set, plan) into a CUDA graph and replayed (one launch per sub-batch instead of ~20:
 // what bounds small real graphs like MuSiQue-1k, where a sweep is a few microseconds of work).  Multi-GPU runs (epoch
-// values change per sweep) and HRAG_PPR_GRAPHS=0 take the plain path.
+// values change per sweep) take the plain path.
 int dev_ppr_mixed(hrag_t* h, const SweepPlan& plan, float alpha, const int* slot_map, const float* Vexact,
                   const void* rhs16, void* x0_dense, const float* scale, const double* vsum, void** X0, void** D) {
     StageTimer tm(h, ST_PPR);
-    if (h->use_graphs < 0) { const char* e = getenv("HRAG_PPR_GRAPHS"); h->use_graphs = e ? atoi(e) : 1; }
-    if (h->world > 1 || !h->use_graphs || h->use_tma == 1) {
+    if (h->world > 1) {
         HRAG_TRY(dev_ppr_mixed_body(h, plan, alpha, slot_map, Vexact, rhs16, x0_dense, scale, vsum, X0, D));
         return p2p_wait(h);     // the consumers of X0 / D (gather kernels) need every peer's last rows
     }
@@ -910,8 +891,7 @@ void hrag_destroy(hrag_t* h) {
                          &h->slot_vid[1], &h->Vc[0], &h->Vc[1], &h->R16[0], &h->R16[1], &h->rho, &h->xr_mm, &h->xr_keys})
         b->release();
     cudaFree(h->g.row_ptr); cudaFree(h->g.cv); cudaFree(h->g.long_rows); cudaFree(h->g.long_seg_ptr);
-    cudaFree(h->g.segs); cudaFree(h->g.seg_partial); cudaFree(h->g.tma_blk_row); cudaFree(h->g.row_order);
-    for (int i = 0; i < 5; ++i) cudaFree(h->g.blk_row[i]);
+    cudaFree(h->g.segs); cudaFree(h->g.seg_partial); cudaFree(h->g.row_order);
     cudaFree(h->t.passage_vid); cudaFree(h->t.fact_subj_vid); cudaFree(h->t.fact_obj_vid);
     cudaFree(h->t.ent_chunk_count);
     for (int i = 0; i < 2; ++i) {
@@ -1002,9 +982,7 @@ int hrag_load_graph_csr(hrag_t* h, int64_t n_nodes, int64_t row_lo, int64_t row_
     PprGraph& g = h->g;
     cudaFree(g.row_ptr); cudaFree(g.cv); cudaFree(g.long_rows); cudaFree(g.long_seg_ptr); cudaFree(g.segs);
     cudaFree(g.seg_partial);
-    cudaFree(g.tma_blk_row);
     cudaFree(g.row_order);
-    for (int i = 0; i < 5; ++i) cudaFree(g.blk_row[i]);
     g = PprGraph();
     g.num_sms = h->num_sms;
     g.n_global = (int)n_nodes;
@@ -1048,35 +1026,10 @@ int hrag_load_graph_csr(hrag_t* h, int64_t n_nodes, int64_t row_lo, int64_t row_
         cv[(size_t)i] = make_int2(col[i], bits);
     }
     HRAG_CUDA(cudaMalloc(&g.row_ptr, (size_t)(n_rows + 1) * sizeof(int)));
-    HRAG_CUDA(cudaMalloc(&g.cv, ((size_t)nnz + 2) * sizeof(int2)));   // +2: bulk copies round up to 16 B
+    HRAG_CUDA(cudaMalloc(&g.cv, ((size_t)nnz + 2) * sizeof(int2)));   // +2 zeroed spares: never null, even with no edges
     HRAG_CUDA(cudaMemset(g.cv, 0, ((size_t)nnz + 2) * sizeof(int2)));
     HRAG_CUDA(cudaMemcpy(g.row_ptr, rp.data(), (size_t)(n_rows + 1) * sizeof(int), cudaMemcpyHostToDevice));
     if (nnz) HRAG_CUDA(cudaMemcpy(g.cv, cv.data(), (size_t)nnz * sizeof(int2), cudaMemcpyHostToDevice));
-    // row blocks of the staged sweep, one partition per batch width (rows per block depends on it)
-    for (int wi = 0; wi < 5; ++wi) {
-        const int lpr = 1 << wi;                       // B = 4 << wi
-        const int max_rows = std::min(2 * (256 / lpr), 256);
-        const int cap = 2048;
-        std::vector<int> blk;
-        int r = 0;
-        while (r < n_rows) {
-            const int deg = rp[r + 1] - rp[r];
-            if (deg > g.long_thresh) { blk.push_back(r | (int)0x80000000); ++r; continue; }
-            const int start = r;
-            int cnt = 0;
-            while (r < n_rows && r - start < max_rows) {
-                const int d = rp[r + 1] - rp[r];
-                if (d > g.long_thresh || cnt + d > cap) break;
-                cnt += d;
-                ++r;
-            }
-            blk.push_back(start);
-        }
-        g.n_blk[wi] = (int)blk.size();
-        blk.push_back(n_rows);
-        HRAG_CUDA(cudaMalloc(&g.blk_row[wi], blk.size() * sizeof(int)));
-        HRAG_CUDA(cudaMemcpy(g.blk_row[wi], blk.data(), blk.size() * sizeof(int), cudaMemcpyHostToDevice));
-    }
     {   // fp16 sweep: within each block of 64 rows (one CTA) order the rows by length so a warp's 8 rows match
         std::vector<int> order(n_rows);
         for (int r = 0; r < n_rows; ++r) order[r] = r;
@@ -1087,13 +1040,6 @@ int hrag_load_graph_csr(hrag_t* h, int64_t n_nodes, int64_t row_lo, int64_t row_
         }
         HRAG_CUDA(cudaMalloc(&g.row_order, std::max<size_t>(1, order.size()) * sizeof(int)));
         if (n_rows) HRAG_CUDA(cudaMemcpy(g.row_order, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice));
-    }
-    {
-        std::vector<int> tb;
-        tma_build_blocks(rp.data(), n_rows, g.long_thresh, tb);
-        g.n_tma_blk = (int)tb.size() - 1;
-        HRAG_CUDA(cudaMalloc(&g.tma_blk_row, tb.size() * sizeof(int)));
-        HRAG_CUDA(cudaMemcpy(g.tma_blk_row, tb.data(), tb.size() * sizeof(int), cudaMemcpyHostToDevice));
     }
     g.n_long = (int)long_rows.size();
     g.n_seg = (int)segs.size();
@@ -1621,36 +1567,12 @@ int hrag_bench_sweep(hrag_t* h, int32_t B, int32_t sweeps, int32_t method, float
     cudaEvent_t e0, e1;
     HRAG_CUDA(cudaEventCreate(&e0));
     HRAG_CUDA(cudaEventCreate(&e1));
-    const char* pe = getenv("HRAG_L2_PERSIST");
-    const double persist = pe ? atof(pe) : 0.0;
-    if (persist > 0.0) {
-        int max_persist = 0, max_win = 0;
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, h->device);
-        cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, h->device);
-        HRAG_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist));
-        fprintf(stderr, "[hrag] L2 persist: max_persist=%d MB max_window=%d MB ratio=%.2f\n", max_persist >> 20,
-                max_win >> 20, persist);
-    }
-    auto set_window = [&](const float* xbuf) {
-        if (persist <= 0.0) return;
-        int max_win = 0;
-        cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, h->device);
-        cudaStreamAttrValue v;
-        memset(&v, 0, sizeof(v));
-        v.accessPolicyWindow.base_ptr = const_cast<float*>(xbuf);
-        v.accessPolicyWindow.num_bytes = std::min<size_t>(bytes, (size_t)max_win);
-        v.accessPolicyWindow.hitRatio = (float)persist;
-        v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        cudaStreamSetAttribute(h->stream, cudaStreamAttributeAccessPolicyWindow, &v);
-    };
     for (int pass = 0; pass < 2; ++pass) {   // pass 0 = warm-up (3 sweeps), pass 1 = timed
         const int n = pass == 0 ? 3 : sweeps;
         if (pass == 1) HRAG_CUDA(cudaEventRecord(e0, h->stream));
         for (int i = 0; i < n; ++i) {
             const float* x = (i & 1) ? C : A;
             float* y = (i & 1) ? A : C;
-            set_window(x);
             if (method == HRAG_PPR_CHEBYSHEV) HRAG_TRY(ppr_sweep(h->g, B, x, V, y, y, 0.5f, 1.07f, nullptr, nullptr, h->stream));
             else HRAG_TRY(ppr_sweep(h->g, B, x, V, nullptr, y, 0.5f, 1.f, nullptr, nullptr, h->stream));
             HRAG_TRY(exchange_rows(h, y, B));
@@ -1682,27 +1604,10 @@ int hrag_plan_sweeps(float damping, float tol, int32_t iters, int32_t batch, int
     return 0;
 }
 
-int hrag_set_tuning(hrag_t* h, int mixed_hint, int use_tma, int sorted_rows, int sweep_shape, int k5_debug) {
+int hrag_set_tuning(hrag_t* h, int k5_debug) {
     HRAG_CHECK(h, "hrag_set_tuning: null handle");
     h->graph_generation += 1;
     if (k5_debug >= 0) h->k5_debug = k5_debug;
-    if (sorted_rows >= 0) set_mixed_sorted_rows(sorted_rows);
-    if (sweep_shape >= 0) {
-        HRAG_CHECK(sweep_shape <= 2, "hrag_set_tuning: sweep_shape in [0, 2]");
-        set_mixed_shape(sweep_shape);
-    }
-    if (mixed_hint >= 0) {
-        HRAG_CHECK(mixed_hint <= 4, "hrag_set_tuning: mixed_hint in [0, 4]");
-        set_mixed_hint(mixed_hint);
-    }
-    if (use_tma >= 0) {
-        h->use_tma = use_tma ? 1 : 0;
-        if (h->use_tma && h->slab) {
-            hrag::Buf* views[5] = {&h->H[0], &h->H[1], &h->H[2], &h->H[3], &h->H0b};
-            for (int i = 0; i < 5; ++i) HRAG_TRY(tma_state_map(views[i]->p, (int64_t)state_rows(h), h->xmap[i]));
-            h->xmaps_valid = true;
-        }
-    }
     return 0;
 }
 

@@ -4,8 +4,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <vector>
-
 namespace hrag {
 
 struct SeedTables;
@@ -28,15 +26,8 @@ struct PprGraph {
     int4* segs = nullptr;         // [n_seg] {local row, begin, end, 0}
     float* seg_partial = nullptr; // [n_seg * Bmax]
     int max_batch = 0;
-    // staged sweep: row blocks (<= 2048 non-zeros, contiguous in cv) per batch width 4<<i;
-    // blk_row[i] has n_blk[i] + 1 entries, bit 31 marks a block that is one long row
-    int* blk_row[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    int n_blk[5] = {0, 0, 0, 0, 0};
     int num_sms = 148;
     int* row_order = nullptr;     // [n_rows] fp16 sweep: rows of each 64-row CTA block sorted by length (desc)
-    // TMA-gather sweep (ppr_tma.cu): row blocks of <= 64 rows / <= 1024 non-zeros, bit 31 = long row
-    int* tma_blk_row = nullptr;
-    int n_tma_blk = 0;
 };
 
 // One sweep  y[i,:] = w * (alpha * sum_j P[i,j] x[j,:] + v[i,:]) + (1 - w) * prev[i,:]
@@ -80,15 +71,6 @@ int mixed_sweep(const PprGraph& g, int mode, const void* xh, const int* slot_map
                 float t, float* partials, int* n_partials, const PeerOut& peers, const SweepSync& sync,
                 cudaStream_t stream);
 int mixed_partial_rows(const PprGraph& g);
-void set_mixed_hint(int hint);
-void set_mixed_shape(int shape);         // gathers in flight per lane / CTAs per SM: 0 = 4/6, 1 = 8/4, 2 = 6/5
-void set_mixed_sorted_rows(int on);   // 1 (default): a warp's 8 rows are picked by length within the CTA's 64-row block   // L2 policy variant of the fp16 sweep (0 none, 1 default, 2, 3)
-// K1t (ppr_tma.cu): the same sweep (mode 0, no column sums, short rows only) with the gathered state rows fetched
-// by TMA gather4 into a shared-memory ring.  map128 = CUtensorMap of the x buffer (tma_state_map).
-int tma_state_map(const void* xh, int64_t n_rows, void* map128);
-void tma_build_blocks(const int* row_ptr, int n_rows, int long_thresh, std::vector<int>& blk);
-int mixed_sweep_tma(const PprGraph& g, const void* map128, const int* slot_map, const void* rhs_h, const void* prevh,
-                    void* yh, float alpha, float w, const PeerOut& peers, cudaStream_t stream);
 // vsum[32] <- column sums of V32 [n_rows, 32] (>= 0; `partials` = scratch of >= 1024*32 floats);
 // scale[b] = 2^floor(log2(32768 (1 - alpha) / vsum[b])) -- overflow-proof, see ppr_mixed.cu;
 // V16 = fp16(scale * V32).

@@ -28,9 +28,9 @@
 //
 // Row walk: 4 gathers in flight per lane, the ragged end of a row is one PREDICATED batch (not a
 // serial tail), and the 64 rows of a CTA are handed to the groups by length (row_order) so the 8
-// rows that share a warp finish together.  Cache-policy variants (createpolicy descriptors on
-// gathers / streams, L1::no_allocate) are kept as template HINTs; plain read-only loads win once
-// the tail is predicated -- profiles/r2_k1m_variants_{a,b,c}.txt.
+// rows that share a warp finish together.  Loads are plain read-only loads: cache-policy
+// descriptors on gathers / streams and L1::no_allocate were measured slower once the tail is
+// predicated -- profiles/r2_k1m_variants_{a,b,c}.txt.
 //
 // K5 (node-range sharding, k_sweep_h_push): each CTA stages its 64 output rows in shared memory
 // and pushes the 4-KB block into every peer GPU's copy of y with one TMA bulk copy per peer over
@@ -78,82 +78,19 @@ __device__ __forceinline__ void fma8(float (&acc)[8], float a, const uint4& u) {
     for (int j = 0; j < 8; ++j) acc[j] = fmaf(a, f[j], acc[j]);
 }
 
-// ---- cache policies -------------------------------------------------------------------------
-// HINT 0: plain read-only loads.  1: gathers L2 evict_last, streams L2 evict_first (createpolicy descriptors).
-// 2: as 1 with only half of the gathered lines marked evict_last.  3: as 1, gathers also bypass L1 allocation.
-// 4: gathers bypass L1 allocation, nothing else (no descriptor: every gathered row is its own line, so L1 holds
-// nothing reusable and is left to the (col, val) stream).  Measured in profiles/r2_k1m_variants*.txt.
-template <int HINT>
-struct Policies {
-    uint64_t keep, stream;
-    __device__ __forceinline__ Policies() {
-        keep = stream = 0;
-        if (HINT == 1 || HINT == 3) asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(keep));
-        if (HINT == 2) asm("createpolicy.fractional.L2::evict_last.L2::evict_unchanged.b64 %0, 0.5;" : "=l"(keep));
-        if (HINT >= 1 && HINT <= 3) asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(stream));
-    }
-};
-// predicated forms: `ok == false` yields zeros without touching memory (the ragged end of a row is a predicated
-// batch); the predicate lives inside the asm so the compiler cannot turn it into a branch
-template <int HINT>
-__device__ __forceinline__ uint4 ld_gather(const uint4* p, bool ok, const Policies<HINT>& pol) {
-    if (HINT == 0) return ok ? __ldg(p) : make_uint4(0u, 0u, 0u, 0u);
-    uint4 v;
-    if (HINT == 4)
-        asm("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %5, 0;\n\t"
-            "mov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
-            "@q ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];\n\t}"
-            : "=&r"(v.x), "=&r"(v.y), "=&r"(v.z), "=&r"(v.w) : "l"(p), "r"((int)ok));
-    else if (HINT == 3)
-        asm("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %6, 0;\n\t"
-            "mov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
-            "@q ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;\n\t}"
-            : "=&r"(v.x), "=&r"(v.y), "=&r"(v.z), "=&r"(v.w) : "l"(p), "l"(pol.keep), "r"((int)ok));
-    else
-        asm("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %6, 0;\n\t"
-            "mov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
-            "@q ld.global.nc.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;\n\t}"
-            : "=&r"(v.x), "=&r"(v.y), "=&r"(v.z), "=&r"(v.w) : "l"(p), "l"(pol.keep), "r"((int)ok));
-    return v;
-}
-template <int HINT>
-__device__ __forceinline__ int2 ld_cv(const int2* p, bool ok, const Policies<HINT>& pol) {
-    if (HINT == 0 || HINT == 4) return ok ? __ldg(p) : make_int2(0, 0);
-    int2 v;
-    asm("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %4, 0;\n\tmov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\t"
-        "@q ld.global.nc.L2::cache_hint.v2.s32 {%0,%1}, [%2], %3;\n\t}"
-        : "=&r"(v.x), "=&r"(v.y) : "l"(p), "l"(pol.stream), "r"((int)ok));
-    return v;
-}
-// read-once operand of the epilogue (rhs, exact v): no L1 allocation, first out of L2
-template <int HINT>
-__device__ __forceinline__ uint4 ld_stream16(const void* p, const Policies<HINT>& pol) {
-    if (HINT == 0 || HINT == 4) return __ldcs(reinterpret_cast<const uint4*>(p));
-    uint4 v;
-    asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
-        : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p), "l"(pol.stream));
-    return v;
-}
-// prev may alias y (in-place Chebyshev): a coherent load, no .nc
-template <int HINT>
-__device__ __forceinline__ uint4 ld_prev(const uint4* p, const Policies<HINT>& pol) {
-    if (HINT == 0 || HINT == 4) return *p;
-    uint4 v;
-    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
-                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p), "l"(pol.stream) : "memory");
-    return v;
-}
-template <int HINT>
-__device__ __forceinline__ void st_y(uint4* p, const uint4& v, const Policies<HINT>& pol) {
-    if (HINT == 0 || HINT == 4) { *p = v; return; }
-    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1,%2,%3,%4}, %5;"
-                 :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "l"(pol.stream) : "memory");
-}
+// ---- loads ----------------------------------------------------------------------------------------
+// predicated: `ok == false` yields zeros without touching memory (the ragged end of a row is a predicated batch)
+__device__ __forceinline__ uint4 ld_gather(const uint4* p, bool ok) { return ok ? __ldg(p) : make_uint4(0u, 0u, 0u, 0u); }
+__device__ __forceinline__ int2 ld_cv(const int2* p, bool ok) { return ok ? __ldg(p) : make_int2(0, 0); }
+// read-once operand of the epilogue (rhs, exact v): streamed, first out of the caches
+__device__ __forceinline__ uint4 ld_stream16(const void* p) { return __ldcs(reinterpret_cast<const uint4*>(p)); }
+// prev may alias y (in-place Chebyshev): a coherent load, no .nc.  A copy, not a reference into global memory:
+// handing h8_to_f the reference directly schedules the sweep's epilogue differently
+__device__ __forceinline__ uint4 ld_prev(const uint4* p) { return *p; }
 
-template <int U, int HINT>
+template <int U>
 __device__ __forceinline__ void group_row_dot_h(const int2* __restrict__ cv, int s, int e,
-                                                const uint4* __restrict__ xh /* + lane */, float (&acc)[8],
-                                                const Policies<HINT>& pol) {
+                                                const uint4* __restrict__ xh /* + lane */, float (&acc)[8]) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) acc[j] = 0.f;
     // U independent 16-byte gathers in flight per lane; the ragged end of the row is a PREDICATED batch, not a
@@ -162,9 +99,9 @@ __device__ __forceinline__ void group_row_dot_h(const int2* __restrict__ cv, int
         int2 c[U];
         uint4 a[U];
 #pragma unroll
-        for (int j = 0; j < U; ++j) c[j] = ld_cv<HINT>(cv + i + j, i + j < e, pol);
+        for (int j = 0; j < U; ++j) c[j] = ld_cv(cv + i + j, i + j < e);
 #pragma unroll
-        for (int j = 0; j < U; ++j) a[j] = ld_gather<HINT>(xh + (size_t)c[j].x * kLPR, i + j < e, pol);
+        for (int j = 0; j < U; ++j) a[j] = ld_gather(xh + (size_t)c[j].x * kLPR, i + j < e);
 #pragma unroll
         for (int j = 0; j < U; ++j) fma8(acc, __int_as_float(c[j].y), a[j]);
     }
@@ -211,19 +148,18 @@ __device__ __forceinline__ void sync_signal(const SweepSync& sy) {
 // MODE 1: y = t * (scale * v32 - x0 + alpha * acc)            (the refinement residual)
 // rhs / v32 are addressed through slot_map (null = dense).  Returns (in out[]) the value as
 // STORED (after fp16 rounding) so column sums match memory; MODE 1 + FINAL returns |value|.
-template <bool CHEB, int MODE, int HINT>
+template <bool CHEB, int MODE>
 __device__ __forceinline__ void row_epilogue_h(float (&acc)[8], int row, int lane, const int* __restrict__ slot_map,
                                                const uint4* __restrict__ rhs_h, const float4* __restrict__ v32,
                                                const float* __restrict__ col_scale, const uint4* x0h,
                                                const uint4* prevh, uint4* yh, float alpha, float w, float t,
-                                               const PeerOut& peers, const Policies<HINT>& pol, float (&out)[8],
-                                               uint4& packed_out) {
+                                               const PeerOut& peers, float (&out)[8], uint4& packed_out) {
     const size_t o = (size_t)row * kLPR + lane;
     const int slot = slot_map ? __ldg(slot_map + row) : row;
     if (MODE == 0) {
         if (slot >= 0) {
             float r[8];
-            h8_to_f(ld_stream16<HINT>(rhs_h + (size_t)slot * kLPR + lane, pol), r);
+            h8_to_f(ld_stream16(rhs_h + (size_t)slot * kLPR + lane), r);
 #pragma unroll
             for (int j = 0; j < 8; ++j) out[j] = fmaf(alpha, acc[j], r[j]);
         } else {
@@ -232,7 +168,7 @@ __device__ __forceinline__ void row_epilogue_h(float (&acc)[8], int row, int lan
         }
         if (CHEB) {
             float p[8];
-            h8_to_f(ld_prev<HINT>(prevh + o, pol), p);
+            h8_to_f(ld_prev(prevh + o), p);
             const float w1 = 1.f - w;
 #pragma unroll
             for (int j = 0; j < 8; ++j) out[j] = fmaf(w, out[j], w1 * p[j]);
@@ -243,7 +179,7 @@ __device__ __forceinline__ void row_epilogue_h(float (&acc)[8], int row, int lan
         float v[8];
         if (slot >= 0) {
             const float4* vp = v32 + ((size_t)slot * kLPR + lane) * 2;
-            const uint4 ua = ld_stream16<HINT>(vp, pol), ub = ld_stream16<HINT>(vp + 1, pol);
+            const uint4 ua = ld_stream16(vp), ub = ld_stream16(vp + 1);
             v[0] = __uint_as_float(ua.x); v[1] = __uint_as_float(ua.y); v[2] = __uint_as_float(ua.z); v[3] = __uint_as_float(ua.w);
             v[4] = __uint_as_float(ub.x); v[5] = __uint_as_float(ub.y); v[6] = __uint_as_float(ub.z); v[7] = __uint_as_float(ub.w);
         } else {
@@ -258,7 +194,7 @@ __device__ __forceinline__ void row_epilogue_h(float (&acc)[8], int row, int lan
     }
     const uint4 packed = f_to_h8(out);
     packed_out = packed;
-    st_y<HINT>(yh + o, packed, pol);
+    yh[o] = packed;
     // K5, direct form (long rows only): the same 16 bytes go into every peer GPU's copy of y.  The main kernel passes
     // no peers here and pushes its whole 4-KB row block at once (below)
 #pragma unroll
@@ -310,10 +246,11 @@ struct SweepArgs {
 // Single-GPU sweep: one block of 64 rows per CTA.  (Kept free of the exchange code of k_sweep_h_push below: sharing one
 // body -- a block loop with the staging / bulk-copy code behind a uniform branch -- cost the plain sweep 13 %:
 // 0.178 vs 0.157 ms on C3, profiles/r2_k1m_variants_d.txt.)
-template <bool CHEB, int MODE, bool FINAL, int U, int MINB, int HINT>
-__global__ void __launch_bounds__(kThreads, MINB)
+// 4 gathers in flight per lane at 6 CTAs per SM (8 / 4 and 6 / 5 measured slower, DESIGN.md section 4).
+template <bool CHEB, int MODE, bool FINAL>
+__global__ void __launch_bounds__(kThreads, 6)
 k_sweep_h(const SweepArgs a) {
-    const Policies<HINT> pol;
+    constexpr int U = 4;
     const int g = threadIdx.x / kLPR, l = threadIdx.x % kLPR;
     const int slot_r = blockIdx.x * kGPB + g;
     float out[8];
@@ -325,9 +262,9 @@ k_sweep_h(const SweepArgs a) {
         if (e - s <= a.long_thresh) {
             float acc[8];
             uint4 packed;
-            group_row_dot_h<U, HINT>(a.cv, s, e, a.xh + l, acc, pol);
-            row_epilogue_h<CHEB, MODE, HINT>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh,
-                                             a.prevh, a.yh, a.alpha, a.w, a.t, PeerOut(), pol, out, packed);
+            group_row_dot_h<U>(a.cv, s, e, a.xh + l, acc);
+            row_epilogue_h<CHEB, MODE>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh,
+                                       a.prevh, a.yh, a.alpha, a.w, a.t, PeerOut(), out, packed);
         }
     }
     if (FINAL) block_colsum_h(out, a.partials + (size_t)blockIdx.x * kB);
@@ -337,7 +274,7 @@ k_sweep_h(const SweepArgs a) {
 template <bool CHEB, int MODE, bool FINAL>
 __global__ void __launch_bounds__(kThreads, 6)
 k_sweep_h_push(const SweepArgs a, const PeerOut peers, const SweepSync sy) {
-    constexpr int U = 4, HINT = 0;
+    constexpr int U = 4;
     // K5 staging: a block's 64 output rows are one contiguous 4-KB piece of y.  They are collected in shared memory and
     // pushed to every peer as ONE bulk copy per peer by the TMA engine (cp.async.bulk shared -> peer global over NVLink,
     // SASS UBLKCP): full-size NVLink packets, no store instructions on the SMs' LSUs, double-buffered so the copy of block
@@ -346,7 +283,6 @@ k_sweep_h_push(const SweepArgs a, const PeerOut peers, const SweepSync sy) {
     __shared__ __align__(128) uint4 s_out[2][kThreads];
     __shared__ unsigned char s_valid[kGPB];
     sync_wait(sy);
-    const Policies<HINT> pol;
     const int g = threadIdx.x / kLPR, l = threadIdx.x % kLPR;
     const bool push = peers.n > 0 && !(sy.debug & 2);    // uniform
     const int n_blocks = (a.n_rows + kGPB - 1) / kGPB;
@@ -370,9 +306,9 @@ k_sweep_h_push(const SweepArgs a, const PeerOut peers, const SweepSync sy) {
             if (e - s <= a.long_thresh) {
                 float acc[8];
                 uint4 packed;
-                group_row_dot_h<U, HINT>(a.cv, s, e, a.xh + l, acc, pol);
-                row_epilogue_h<CHEB, MODE, HINT>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh,
-                                                 a.prevh, a.yh, a.alpha, a.w, a.t, PeerOut(), pol, out, packed);
+                group_row_dot_h<U>(a.cv, s, e, a.xh + l, acc);
+                row_epilogue_h<CHEB, MODE>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh,
+                                           a.prevh, a.yh, a.alpha, a.w, a.t, PeerOut(), out, packed);
                 if (push) {
                     const int rl = r - blk * kGPB;       // row_order permutes rows inside their own 64-row block only
                     s_out[buf][rl * kLPR + l] = packed;
@@ -447,7 +383,6 @@ __global__ void __launch_bounds__(kThreads)
 k_sweep_long_finalize_h(int n_long, const int* __restrict__ long_rows, const int* __restrict__ long_seg_ptr,
                         const float* __restrict__ seg_partial, const SweepArgs a, const PeerOut peers,
                         const SweepSync sy) {
-    const Policies<0> pol;
     const int g = threadIdx.x / kLPR, l = threadIdx.x % kLPR;
     const int k = blockIdx.x * kGPB + g;
     float out[8];
@@ -462,8 +397,8 @@ k_sweep_long_finalize_h(int n_long, const int* __restrict__ long_rows, const int
 #pragma unroll
             for (int j = 0; j < 8; ++j) acc[j] += seg_partial[(size_t)s * kB + l * 8 + j];
         uint4 packed;
-        row_epilogue_h<CHEB, MODE, 0>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh, a.prevh,
-                                      a.yh, a.alpha, a.w, a.t, peers, pol, out, packed);
+        row_epilogue_h<CHEB, MODE>(acc, a.row_base + r, l, a.slot_map, a.rhs_h, a.v32, a.col_scale, a.xh, a.prevh,
+                                   a.yh, a.alpha, a.w, a.t, peers, out, packed);
     }
     if (FINAL) block_colsum_h(out, a.partials + (size_t)blockIdx.x * kB);
     sync_signal(sy);
@@ -684,28 +619,7 @@ k_state_to_scores_mixed(const __half* __restrict__ X0, const __half* __restrict_
     out[(size_t)b * N + n] = __fdiv_rn(z, (float)(sum0[b] + (double)inv_t * sum1[b]));
 }
 
-int g_mixed_hint = -1;
-int mixed_hint() {   // HRAG_MIXED_HINT / hrag_set_tuning: L2 policy variant of k_sweep_h (see Policies<>)
-    if (g_mixed_hint < 0) { const char* e = getenv("HRAG_MIXED_HINT"); g_mixed_hint = e ? atoi(e) : 0; }
-    return g_mixed_hint;
-}
-
 }  // namespace
-
-void set_mixed_hint(int hint) { g_mixed_hint = hint; }
-static int g_sorted_rows = -1;
-static int mixed_sorted_rows() {
-    if (g_sorted_rows < 0) { const char* e = getenv("HRAG_MIXED_SORTED"); g_sorted_rows = e ? atoi(e) : 1; }
-    return g_sorted_rows;
-}
-void set_mixed_sorted_rows(int on) { g_sorted_rows = on ? 1 : 0; }
-// gathers in flight per lane / CTAs per SM of k_sweep_h: 0 = 4 / 6 (default), 1 = 8 / 4, 2 = 6 / 5
-static int g_shape = -1;
-static int mixed_shape() {
-    if (g_shape < 0) { const char* e = getenv("HRAG_MIXED_SHAPE"); g_shape = e ? atoi(e) : 0; }
-    return g_shape;
-}
-void set_mixed_shape(int shape) { g_shape = shape; }
 
 int mixed_partial_rows(const PprGraph& g) {
     return (int)ceil_div(g.n_rows, kGPB) + (g.n_long ? (int)ceil_div(g.n_long, kGPB) : 0);
@@ -736,7 +650,7 @@ int mixed_sweep(const PprGraph& g, int mode, const void* xh, const int* slot_map
     const int nb_long = g.n_long ? (int)ceil_div(g.n_long, kGPB) : 0;
     SweepArgs a;
     a.n_rows = g.n_rows; a.row_base = g.row_lo; a.long_thresh = g.long_thresh;
-    a.row_order = mixed_sorted_rows() ? g.row_order : nullptr;
+    a.row_order = g.row_order;
     a.row_ptr = g.row_ptr; a.cv = g.cv;
     a.xh = reinterpret_cast<const uint4*>(xh);
     a.slot_map = slot_map;
@@ -774,23 +688,11 @@ int mixed_sweep(const PprGraph& g, int mode, const void* xh, const int* slot_map
     }
     SweepArgs al = a;
     al.partials = fin ? partials + (size_t)nb_rows * kB : nullptr;
-    const int hint = mixed_hint();
-    const int shape = mixed_shape();
-#define HRAG_LAUNCH_HH(C, M, F, U, B, H)                                                                          \
-    k_sweep_h<C, M, F, U, B, H><<<grid_rows, kThreads, 0, st>>>(a)
 #define HRAG_LAUNCH_H(C, M, F)                                                                                    \
     do {                                                                                                          \
         if (nb_rows) {                                                                                            \
             if (sharded) k_sweep_h_push<C, M, F><<<grid_rows, kThreads, 0, st>>>(a, peers, sy);                    \
-            else if (shape == 1 && hint == 4) HRAG_LAUNCH_HH(C, M, F, 8, 4, 4);                                   \
-            else if (shape == 1) HRAG_LAUNCH_HH(C, M, F, 8, 4, 0);                                                \
-            else if (shape == 2 && hint == 4) HRAG_LAUNCH_HH(C, M, F, 6, 5, 4);                                   \
-            else if (shape == 2) HRAG_LAUNCH_HH(C, M, F, 6, 5, 0);                                                \
-            else if (hint == 1) HRAG_LAUNCH_HH(C, M, F, 4, 6, 1);                                                 \
-            else if (hint == 2) HRAG_LAUNCH_HH(C, M, F, 4, 6, 2);                                                 \
-            else if (hint == 3) HRAG_LAUNCH_HH(C, M, F, 4, 6, 3);                                                 \
-            else if (hint == 4) HRAG_LAUNCH_HH(C, M, F, 4, 6, 4);                                                 \
-            else HRAG_LAUNCH_HH(C, M, F, 4, 6, 0);                                                                \
+            else k_sweep_h<C, M, F><<<grid_rows, kThreads, 0, st>>>(a);                                           \
             count_launch();                                                                                       \
         }                                                                                                         \
         if (nb_long) {                                                                                            \
@@ -806,7 +708,6 @@ int mixed_sweep(const PprGraph& g, int mode, const void* xh, const int* slot_map
     else if (fin) HRAG_LAUNCH_H(false, 0, true);
     else HRAG_LAUNCH_H(false, 0, false);
 #undef HRAG_LAUNCH_H
-#undef HRAG_LAUNCH_HH
     if ((nb_rows + nb_long == 0 || trailing_signal) && sy.flags != nullptr) HRAG_TRY(epoch_signal(sy_full, st));
     if (n_partials) *n_partials = nb_rows + nb_long;
     HRAG_CUDA(cudaGetLastError());

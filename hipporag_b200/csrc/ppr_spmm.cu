@@ -22,9 +22,6 @@
 //
 // Roofline (DESIGN.md): HBM-bound; algorithmic bytes per sweep =
 //     nnz * 8 + (n_rows + 1) * 4 + 3 * n_rows * B * 4.
-#include <algorithm>
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 
@@ -189,138 +186,6 @@ k_sweep_long_finalize(int n_long, int row_base, const int* __restrict__ long_row
     if (FINAL) block_colsum<LPR>(out, partials + (size_t)blockIdx.x * (LPR * 4));
 }
 
-
-// ---- staged variant: persistent CTAs, (col,val) stream of a row block staged in shared memory ----
-// A row block = consecutive rows whose non-zeros (<= kStageCap entries) are ONE contiguous byte
-// range of cv[], fetched by one cp.async.bulk (TMA 1-D bulk copy) that completes on an mbarrier.
-// Two stages: the copy of block i+1 is in flight while the CTA gathers for block i, so a row's
-// gathers no longer wait for its (col,val) loads -- ncu showed the plain kernel latency-bound
-// on exactly that dependency (profiles/r1_k1_fp32_sweep_ncu.md).
-constexpr int kStageCap = 2048;                  // cv entries per stage (16 KB)
-constexpr int kStageEntries = kStageCap + 2;     // +2: 16-byte alignment slack at both ends
-
-__device__ __forceinline__ uint32_t smem_addr_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t"
-        "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
-template <int LPR, int U>
-__device__ __forceinline__ float4 group_row_dot_smem(const int2* cvs /* smem, already offset */, int s, int e,
-                                                     const float4* __restrict__ x4 /* + lane */) {
-    float4 acc = f4_zero();
-    int i = s;
-    for (; i + U <= e; i += U) {      // U independent gathers in flight per lane
-        int2 c[U];
-        float4 a[U];
-#pragma unroll
-        for (int j = 0; j < U; ++j) c[j] = cvs[i + j];
-#pragma unroll
-        for (int j = 0; j < U; ++j) a[j] = __ldg(x4 + (size_t)c[j].x * LPR);
-#pragma unroll
-        for (int j = 0; j < U; ++j) f4_fma(acc, __int_as_float(c[j].y), a[j]);
-    }
-    if (U == 8 && i + 4 <= e) {
-        int2 c[4];
-        float4 a[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) c[j] = cvs[i + j];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) a[j] = __ldg(x4 + (size_t)c[j].x * LPR);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) f4_fma(acc, __int_as_float(c[j].y), a[j]);
-        i += 4;
-    }
-    {   // tail of 0..3: predicated, all loads issued before any use
-        int2 c[3];
-        float4 a[3];
-#pragma unroll
-        for (int j = 0; j < 3; ++j) c[j] = (i + j < e) ? cvs[i + j] : make_int2(0, 0);
-#pragma unroll
-        for (int j = 0; j < 3; ++j) a[j] = (i + j < e) ? __ldg(x4 + (size_t)c[j].x * LPR) : f4_zero();
-#pragma unroll
-        for (int j = 0; j < 3; ++j) f4_fma(acc, __int_as_float(c[j].y), a[j]);
-    }
-    return acc;
-}
-
-// minBlocks is given explicitly: without it ptxas schedules for maximum occupancy and interleaves
-// every gather with its FMAs (2-3 loads in flight); with it the U gathers issue back to back.
-template <int LPR, int U, bool CHEB, bool FINAL>
-__global__ void __launch_bounds__(kThreads, (U == 8 ? 3 : 5))
-k_sweep_staged(int n_blk, const int* __restrict__ blk_row /* [n_blk+1], bit31 = long-row block */, int row_base,
-               const int* __restrict__ row_ptr, const int2* __restrict__ cv, const float4* __restrict__ x4,
-               const float4* __restrict__ v4, const float4* prev4, float4* y4, float alpha, float w,
-               float* __restrict__ partials) {
-    constexpr int G = kThreads / LPR;
-    __shared__ __align__(16) int2 stage_buf[2][kStageEntries];
-    __shared__ __align__(8) unsigned long long bars[2];
-    const int g = threadIdx.x / LPR, l = threadIdx.x % LPR;
-    if (threadIdx.x == 0) {
-        mbar_init(smem_addr_u32(&bars[0]), 1);
-        mbar_init(smem_addr_u32(&bars[1]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    auto issue = [&](int blk, int st) {   // thread 0: start the bulk copy of block `blk` into stage `st`
-        const int r0 = __ldg(blk_row + blk), r1 = __ldg(blk_row + blk + 1) & 0x7fffffff;
-        const uint32_t bar = smem_addr_u32(&bars[st]);
-        if (r0 < 0) { mbar_arrive(bar); return; }              // long-row block: nothing to stage
-        const int s = __ldg(row_ptr + r0) & ~1, e = (__ldg(row_ptr + r1) + 1) & ~1;
-        const uint32_t bytes = (uint32_t)(e - s) * 8u;
-        if (bytes == 0) { mbar_arrive(bar); return; }
-        mbar_expect_tx(bar, bytes);
-        bulk_copy_g2s(smem_addr_u32(&stage_buf[st][0]), cv + s, bytes, bar);
-    };
-
-    float4 total = f4_zero();
-    int it = 0;
-    if (threadIdx.x == 0 && (int)blockIdx.x < n_blk) issue(blockIdx.x, 0);
-    for (int blk = blockIdx.x; blk < n_blk; blk += gridDim.x, ++it) {
-        const int st = it & 1;
-        if (threadIdx.x == 0 && blk + (int)gridDim.x < n_blk) issue(blk + gridDim.x, st ^ 1);
-        const int r0 = __ldg(blk_row + blk), r1 = __ldg(blk_row + blk + 1) & 0x7fffffff;
-        if (r0 >= 0) {
-            // row extents of this group's rows first (independent of the staged data)
-            const int base = __ldg(row_ptr + r0) & ~1;
-            mbar_wait(smem_addr_u32(&bars[st]), (uint32_t)((it >> 1) & 1));
-            const int2* cvs = &stage_buf[st][0] - base;
-            for (int r = r0 + g; r < r1; r += G) {
-                const int s = __ldg(row_ptr + r), e = __ldg(row_ptr + r + 1);
-                const float4 acc = group_row_dot_smem<LPR, U>(cvs, s, e, x4 + l);
-                const float4 out = row_epilogue<LPR, CHEB>(acc, (size_t)(row_base + r) * LPR + l, v4, prev4, y4,
-                                                           alpha, w);
-                if (FINAL) f4_add(total, out);
-            }
-        } else {
-            mbar_wait(smem_addr_u32(&bars[st]), (uint32_t)((it >> 1) & 1));
-        }
-        __syncthreads();     // everyone is done with stage st before it is refilled two blocks later
-    }
-    if (FINAL) block_colsum<LPR>(total, partials + (size_t)blockIdx.x * (LPR * 4));
-}
-
 __global__ void __launch_bounds__(256)
 k_colsum_reduce(const float* __restrict__ partials, int n_partials, int B, double* __restrict__ sums) {
     // one CTA per column; fp64 accumulation (an fp32 running sum over 10^4 partials costs ~1e-6)
@@ -337,89 +202,9 @@ k_colsum_reduce(const float* __restrict__ partials, int n_partials, int B, doubl
     if (threadIdx.x == 0) sums[b] = s[0];
 }
 
-// 0 (default) = one row group per slot, (col,val) read through L1; 1 = persistent CTAs with the
-// (col,val) stream staged in shared memory by cp.async.bulk.  Measured on B200 (C3, B=16):
-// 0.140 ms vs 0.144-0.159 ms per sweep -- both sit on the same L1TEX wavefront bound, see DESIGN.md.
-int sweep_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HRAG_PPR_VARIANT");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
-int sweep_unroll() {   // gathers in flight per lane in the staged kernel: 8 (default) or 4
-    static int u = -1;
-    if (u < 0) {
-        const char* e = getenv("HRAG_PPR_UNROLL");
-        u = (e && atoi(e) == 4) ? 4 : 8;
-    }
-    return u;
-}
-
-template <int LPR, int U>
-int staged_grid(int num_sms) {
-    static int per_sm = 0;
-    if (per_sm == 0) {
-        int a = 0, b = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k_sweep_staged<LPR, U, true, true>, kThreads, 0);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_sweep_staged<LPR, U, false, false>, kThreads, 0);
-        per_sm = std::max(1, std::min(a, b));
-    }
-    return per_sm * num_sms;
-}
-
-template <int LPR, int U>
-int launch_sweep_staged(const PprGraph& g, const float* x, const float* v, const float* prev, float* y,
-                        float alpha, float w, float* partials, int* n_partials, cudaStream_t st) {
-    constexpr int GPB = kThreads / LPR;
-    constexpr int WI = LPR == 1 ? 0 : LPR == 2 ? 1 : LPR == 4 ? 2 : LPR == 8 ? 3 : 4;
-    const bool cheb = prev != nullptr;
-    const bool fin = partials != nullptr;
-    const int grid = std::min(staged_grid<LPR, U>(g.num_sms), std::max(g.n_blk[WI], 1));
-    const int nb_long = g.n_long ? (int)ceil_div(g.n_long, GPB) : 0;
-    const float4* x4 = reinterpret_cast<const float4*>(x);
-    const float4* v4 = reinterpret_cast<const float4*>(v);
-    const float4* p4 = reinterpret_cast<const float4*>(prev);
-    float4* y4 = reinterpret_cast<float4*>(y);
-    if (g.n_long) {
-        k_sweep_long_segments<LPR><<<(unsigned)ceil_div((int64_t)g.n_seg * 32, kThreads), kThreads, 0, st>>>(
-            g.n_seg, g.segs, g.cv, x4, reinterpret_cast<float4*>(g.seg_partial));
-        count_launch();
-    }
-    float* part_long = fin ? partials + (size_t)grid * LPR * 4 : nullptr;
-#define HRAG_LAUNCH_ST(C, F)                                                                           \
-    do {                                                                                               \
-        k_sweep_staged<LPR, U, C, F><<<grid, kThreads, 0, st>>>(g.n_blk[WI], g.blk_row[WI], g.row_lo,     \
-                                                             g.row_ptr, g.cv, x4, v4, p4, y4, alpha, w, \
-                                                             partials);                                \
-        count_launch();                                                                                \
-        if (nb_long) {                                                                                 \
-            k_sweep_long_finalize<LPR, C, F><<<nb_long, kThreads, 0, st>>>(                            \
-                g.n_long, g.row_lo, g.long_rows, g.long_seg_ptr,                                       \
-                reinterpret_cast<const float4*>(g.seg_partial), v4, p4, y4, alpha, w, part_long);      \
-            count_launch();                                                                            \
-        }                                                                                              \
-    } while (0)
-    if (cheb && fin) HRAG_LAUNCH_ST(true, true);
-    else if (cheb) HRAG_LAUNCH_ST(true, false);
-    else if (fin) HRAG_LAUNCH_ST(false, true);
-    else HRAG_LAUNCH_ST(false, false);
-#undef HRAG_LAUNCH_ST
-    if (n_partials) *n_partials = grid + nb_long;
-    HRAG_CUDA(cudaGetLastError());
-    return 0;
-}
-
 template <int LPR>
 int launch_sweep(const PprGraph& g, const float* x, const float* v, const float* prev, float* y, float alpha,
                  float w, float* partials, int* n_partials, cudaStream_t st) {
-    if (sweep_variant() == 1 && g.blk_row[0] != nullptr) {
-        if (sweep_unroll() == 8)
-            return launch_sweep_staged<LPR, 8>(g, x, v, prev, y, alpha, w, partials, n_partials, st);
-        return launch_sweep_staged<LPR, 4>(g, x, v, prev, y, alpha, w, partials, n_partials, st);
-    }
     constexpr int GPB = kThreads / LPR;
     const bool cheb = prev != nullptr;
     const bool fin = partials != nullptr;
@@ -462,10 +247,9 @@ int launch_sweep(const PprGraph& g, const float* x, const float* v, const float*
 
 }  // namespace
 
-int ppr_sweep_partial_rows(const PprGraph& g, int B) {   // upper bound over both kernel variants
+int ppr_sweep_partial_rows(const PprGraph& g, int B) {
     const int GPB = kThreads / (B / 4);
-    const int rows = std::max((int)ceil_div(g.n_rows, GPB), 32 * g.num_sms);
-    return rows + (g.n_long ? (int)ceil_div(g.n_long, GPB) : 0);
+    return (int)ceil_div(g.n_rows, GPB) + (g.n_long ? (int)ceil_div(g.n_long, GPB) : 0);
 }
 
 int ppr_sweep(const PprGraph& g, int B, const float* x, const float* v, const float* prev, float* y,

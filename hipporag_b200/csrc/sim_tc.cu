@@ -24,7 +24,6 @@
 #include <cuda_bf16.h>
 
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -135,7 +134,6 @@ struct TcParams {
     // fused epilogue (FUSE): per (query, n-tile) min/max and the 8 best rank keys instead of scores
     float2* part_mm;          // [Bq, num_n_tiles]
     uint64_t* part_keys;      // [Bq, num_n_tiles, 8]
-    int debug_mode;           // 0 = normal; 1 = TMA only (no MMAs issued); 2 = MMA only (no TMA loads) -- timing probes
     // threshold epilogue (FUSE == 2, index-time synonymy KNN): every score >= thr is appended to its query's
     // candidate list as a rank key; cand_count keeps counting past cand_cap so overflow is detectable
     float thr;
@@ -214,7 +212,6 @@ k_sim_tc(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ C
                 }
                 for (int kb = 0; kb < nkb; ++kb) {
                     mbar_wait(empty_bar(stage), phase ^ 1u);
-                    if (p.debug_mode == 2) { mbar_arrive(full_bar(stage)); if (++stage == STAGES) { stage = 0; phase ^= 1u; } continue; }
                     mbar_expect_tx(full_bar(stage), STAGE_BYTES);
                     const uint32_t sa = base + stage * STAGE_BYTES;
                     tma_load_2d(sa, &map_q_hi, full_bar(stage), kb * BKs, mt * BM);
@@ -243,9 +240,7 @@ k_sim_tc(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ C
                     tc_fence_after();
                     const uint32_t sa = base + stage * STAGE_BYTES;
                     const uint64_t a_hi = umma_desc_kmajor<ROW_BYTES>(sa), b_hi = umma_desc_kmajor<ROW_BYTES>(sa + OFF_B_HI);
-                    if (p.debug_mode == 1) {
-                        // probe: no MMAs; the commits below complete immediately
-                    } else if (SPLIT) {
+                    if (SPLIT) {
                         const uint64_t a_lo = umma_desc_kmajor<ROW_BYTES>(sa + OFF_A_LO);
                         const uint64_t b_lo = umma_desc_kmajor<ROW_BYTES>(sa + OFF_B_LO);
                         // smallest terms first: lo.lo, hi.lo, lo.hi, then hi.hi
@@ -368,253 +363,6 @@ k_sim_tc(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ C
     }
 }
 
-// ================================================================================================
-// 2-CTA variant of the split GEMM (tcgen05 cta_group::2).  A pair of CTAs on one TPC computes a
-// 256-query x 256-embedding tile: each CTA keeps its own 128 query rows (A) and loads only HALF of the
-// embedding tile (128 of the 256 B rows); the MMA unit reads both halves.  Per SM that is 32 KB of
-// operands per stage instead of 48 KB for the same MMA time and the 192-KB ring holds 6 stages instead
-// of 4.  Correct (same parity tests) but measured SLOWER than the 1-CTA kernel on B200 (221 vs 195 ms,
-// DESIGN.md section 4), so it is kept selectable (HRAG_SIM_2CTA=1) and is not the default.
-// Protocol: both CTAs' TMA loads complete on the LEADER's full barrier (count 2: leader arrive.expect_tx
-// + peer remote arrive); the leader's single MMA thread issues cta_group::2 MMAs and multicasts its
-// commits to both CTAs' empty / tmem-full barriers; the 8 epilogue warps of the pair arrive on the
-// leader's tmem-empty barrier.
-// ================================================================================================
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t local_addr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0,
-                                                int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t smem_dst, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols));
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {   // arrives on `bar` in BOTH CTAs of the pair
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                              uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-}
-// kind::f16, D fp32, A/B bf16 K-major, N = 256, M = 256 (128 rows per CTA)
-constexpr uint32_t kIdesc2 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)((2 * BM) >> 4) << 24);
-
-template <bool FUSE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
-k_sim_tc2(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ CUtensorMap map_q_lo,
-          const __grid_constant__ CUtensorMap map_e_hi /* box 32 x 128 */,
-          const __grid_constant__ CUtensorMap map_e_lo, TcParams p) {
-    constexpr int STAGES = 6;
-    constexpr int BKs = BK / 2, ROW_BYTES = BKs * 2;               // 32 K-columns, 64-byte swizzle rows
-    constexpr int A_BYTES = BM * ROW_BYTES;                        // 8 KB: this CTA's 128 query rows (hi or lo)
-    constexpr int BH_BYTES = (BN / 2) * ROW_BYTES;                 // 8 KB: this CTA's half of the embedding tile
-    constexpr int STAGE_BYTES = 2 * (A_BYTES + BH_BYTES);          // 32 KB  [A_hi | A_lo | B_hi | B_lo]
-    constexpr int OFF_A_LO = A_BYTES, OFF_B_HI = 2 * A_BYTES, OFF_B_LO = 2 * A_BYTES + BH_BYTES;
-    static_assert(STAGES * STAGE_BYTES == RING_BYTES, "ring size");
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t raw = smem_u32(smem_raw);
-    const uint32_t base = (raw + 1023u) & ~1023u;
-    const uint32_t bars = base + RING_BYTES;
-    auto full_bar = [&](int s) { return bars + 8u * s; };           // used in the leader only
-    auto empty_bar = [&](int s) { return bars + 64u + 8u * s; };
-    auto tfull_bar = [&](int a) { return bars + 128u + 8u * a; };
-    auto tempty_bar = [&](int a) { return bars + 160u + 8u * a; };  // used in the leader only
-    const uint32_t tmem_slot = bars + 192u;
-    volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw));
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const bool leader = rank == 0;
-    const int nkb = (p.dim + BKs - 1) / BKs;
-    const int num_mp = (p.Bq + 2 * BM - 1) / (2 * BM);             // 256-query tiles
-    const int total = num_mp * p.num_n_tiles;
-    const int cluster_id = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_q_hi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_q_lo) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_e_hi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_e_lo) : "memory");
-    }
-    if (warp == 1) {
-        if (lane == 0) {
-            for (int s = 0; s < STAGES; ++s) { mbar_init(full_bar(s), 2); mbar_init(empty_bar(s), 1); }
-            for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 8); }
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncwarp();
-        tmem_alloc_2sm(tmem_slot, TMEM_COLS);
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();            // peer barriers are initialised before anyone signals them
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot_ptr;
-
-    if (warp == 0) {
-        // ===== TMA producer (one per CTA): own query rows + own half of the embedding tile =====
-        if (lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int w = cluster_id; w < total; w += n_clusters) {
-                const int mp = w % num_mp, nt = w / num_mp;
-                const int row_a = mp * 2 * BM + (int)rank * BM;
-                const int row_b = nt * BN + (int)rank * (BN / 2);
-                for (int kb = 0; kb < nkb; ++kb) {
-                    mbar_wait(empty_bar(stage), phase ^ 1u);
-                    const uint32_t lbar = mapa_u32(full_bar(stage), 0);
-                    if (leader) mbar_expect_tx(full_bar(stage), 2 * STAGE_BYTES);
-                    else mbar_arrive_cluster(lbar);
-                    const uint32_t sa = base + stage * STAGE_BYTES;
-                    tma_load_2d_2sm(sa, &map_q_hi, lbar, kb * BKs, row_a);
-                    tma_load_2d_2sm(sa + OFF_A_LO, &map_q_lo, lbar, kb * BKs, row_a);
-                    tma_load_2d_2sm(sa + OFF_B_HI, &map_e_hi, lbar, kb * BKs, row_b);
-                    tma_load_2d_2sm(sa + OFF_B_LO, &map_e_lo, lbar, kb * BKs, row_b);
-                    if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer: one thread of the LEADER CTA drives both tensor cores =====
-        if (leader && lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0;
-            int acc = 0;
-            uint32_t acc_phase = 0;
-            for (int w = cluster_id; w < total; w += n_clusters) {
-                mbar_wait(tempty_bar(acc), acc_phase ^ 1u);      // both CTAs' epilogues drained this accumulator
-                tc_fence_after();
-                const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
-                for (int kb = 0; kb < nkb; ++kb) {
-                    mbar_wait(full_bar(stage), phase);
-                    tc_fence_after();
-                    const uint32_t sa = base + stage * STAGE_BYTES;
-                    const uint64_t a_hi = umma_desc_kmajor<ROW_BYTES>(sa), a_lo = umma_desc_kmajor<ROW_BYTES>(sa + OFF_A_LO);
-                    const uint64_t b_hi = umma_desc_kmajor<ROW_BYTES>(sa + OFF_B_HI);
-                    const uint64_t b_lo = umma_desc_kmajor<ROW_BYTES>(sa + OFF_B_LO);
-#pragma unroll
-                    for (int k = 0; k < BKs / UK; ++k)
-                        umma_bf16_2sm(tmem_d, a_lo + (uint64_t)(2 * k), b_lo + (uint64_t)(2 * k), kIdesc2,
-                                      (kb > 0 || k > 0) ? 1u : 0u);
-#pragma unroll
-                    for (int k = 0; k < BKs / UK; ++k)
-                        umma_bf16_2sm(tmem_d, a_hi + (uint64_t)(2 * k), b_lo + (uint64_t)(2 * k), kIdesc2, 1u);
-#pragma unroll
-                    for (int k = 0; k < BKs / UK; ++k)
-                        umma_bf16_2sm(tmem_d, a_lo + (uint64_t)(2 * k), b_hi + (uint64_t)(2 * k), kIdesc2, 1u);
-#pragma unroll
-                    for (int k = 0; k < BKs / UK; ++k)
-                        umma_bf16_2sm(tmem_d, a_hi + (uint64_t)(2 * k), b_hi + (uint64_t)(2 * k), kIdesc2, 1u);
-                    umma_commit_2sm(empty_bar(stage));           // frees the slot in both CTAs
-                    if (kb == nkb - 1) umma_commit_2sm(tfull_bar(acc));
-                    if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-                }
-                if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
-            }
-        }
-    } else {
-        // ===== epilogue (both CTAs): warps 2..5, TMEM lane quarter = warp % 4 =====
-        const int quarter = warp & 3;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (int w = cluster_id; w < total; w += n_clusters) {
-            const int mp = w % num_mp, nt = w / num_mp;
-            mbar_wait(tfull_bar(acc), acc_phase);
-            tc_fence_after();
-            const int q = mp * 2 * BM + (int)rank * BM + quarter * 32 + lane;
-            const int64_t n0 = (int64_t)nt * BN;
-            if (FUSE) {
-                float mn = INFINITY, mx = -INFINITY;
-                uint64_t best[kFuseK];
-#pragma unroll
-                for (int j = 0; j < kFuseK; ++j) best[j] = 0ull;
-#pragma unroll 1
-                for (int c = 0; c < BN / 32; ++c) {
-                    uint32_t r[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + c * 32), r);
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const int64_t col = n0 + c * 32 + j;
-                        if (col < p.M) {
-                            const float f = __uint_as_float(r[j]);
-                            mn = fminf(mn, f);
-                            mx = fmaxf(mx, f);
-                            uint64_t key = rank_key(f, (uint32_t)col);
-                            if (key > best[kFuseK - 1]) {
-#pragma unroll
-                                for (int k = 0; k < kFuseK; ++k)
-                                    if (key > best[k]) { const uint64_t tmp = best[k]; best[k] = key; key = tmp; }
-                            }
-                        }
-                    }
-                }
-                if (q < p.Bq) {
-                    const size_t o = (size_t)q * p.num_n_tiles + nt;
-                    p.part_mm[o] = make_float2(mn, mx);
-#pragma unroll
-                    for (int k = 0; k < kFuseK; k += 2)
-                        *reinterpret_cast<ulonglong2*>(p.part_keys + o * kFuseK + k) = make_ulonglong2(best[k], best[k + 1]);
-                }
-            } else {
-                float* row = p.S + (size_t)q * p.ldS + n0;
-#pragma unroll 1
-                for (int c = 0; c < BN / 32; ++c) {
-                    uint32_t r[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + c * 32), r);
-                    if (q < p.Bq) {
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4) {
-                            if (n0 + c * 32 + j < p.ldS)
-                                *reinterpret_cast<float4*>(row + c * 32 + j) =
-                                    make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]),
-                                                __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3]));
-                        }
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(mapa_u32(tempty_bar(acc), 0));
-            if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();            // nobody frees TMEM / exits while the pair still uses its smem or barriers
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc_2sm(tmem_base, TMEM_COLS);
-    }
-}
-
 // x = hi + lo with hi = bf16(x), lo = bf16(x - hi)
 __global__ void __launch_bounds__(256)
 k_split_bf16(const float* __restrict__ x, int64_t n, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
@@ -705,7 +453,6 @@ int sim_tc_threshold(const void* q_hi, const void* q_lo, int Bq, const void* e_h
     HRAG_TRY(make_map(&mel, e_lo, M, dim, bkc, BN));
     TcParams p;
     p.Bq = Bq; p.M = M; p.dim = dim; p.S = nullptr; p.ldS = 0; p.part_mm = nullptr; p.part_keys = nullptr;
-    p.debug_mode = 0;
     p.thr = thr; p.cand_keys = cand_keys; p.cand_count = cand_count; p.cand_cap = cand_cap;
     p.num_m_tiles = (int)ceil_div(Bq, BM);
     p.num_n_tiles = (int)ceil_div(M, BN);
@@ -728,8 +475,6 @@ int sim_tc(const void* q_hi, const void* q_lo, int Bq, const void* e_hi, const v
         HRAG_CUDA(cudaFuncSetAttribute(k_sim_tc<false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
         HRAG_CUDA(cudaFuncSetAttribute(k_sim_tc<true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
         HRAG_CUDA(cudaFuncSetAttribute(k_sim_tc<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-        HRAG_CUDA(cudaFuncSetAttribute(k_sim_tc2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-        HRAG_CUDA(cudaFuncSetAttribute(k_sim_tc2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
         attr_set = true;
     }
     CUtensorMap mqh, mql, meh, mel;
@@ -741,32 +486,11 @@ int sim_tc(const void* q_hi, const void* q_lo, int Bq, const void* e_hi, const v
     TcParams p;
     p.Bq = Bq; p.M = M; p.dim = dim; p.S = S; p.ldS = ldS; p.part_mm = part_mm; p.part_keys = part_keys;
     const bool fuse = part_mm != nullptr;
-    p.debug_mode = 0;
     p.thr = 0.f; p.cand_keys = nullptr; p.cand_count = nullptr; p.cand_cap = 0;
-    if (const char* ed = getenv("HRAG_SIM_DEBUG")) p.debug_mode = atoi(ed);
     HRAG_CHECK(fuse || (S != nullptr && ldS % 4 == 0), "sim_tc: score buffer missing");
     p.num_m_tiles = (int)ceil_div(Bq, BM);
     p.num_n_tiles = (int)ceil_div(M, BN);
-    const int64_t tiles = (int64_t)p.num_m_tiles * p.num_n_tiles;
-    int grid = (int)std::min<int64_t>(tiles, num_sms);
-    if (const char* eg = getenv("HRAG_SIM_GRID")) grid = std::max(1, std::min(grid, atoi(eg)));   // experiment knob
-    // HRAG_SIM_2CTA=1 selects the cta_group::2 kernel.  Measured on B200 (C3 stage A, 10k queries): 221 ms
-    // vs 195 ms for the 1-CTA kernel -- fewer operand bytes per SM did not help, so it is not the default.
-    static int use_2cta = -1;
-    if (use_2cta < 0) { const char* e2 = getenv("HRAG_SIM_2CTA"); use_2cta = e2 ? atoi(e2) : 0; }
-    if (n_seg == 4 && use_2cta && num_sms >= 2) {
-        CUtensorMap meh2, mel2;                                  // embedding maps with a 128-row box (half tile)
-        HRAG_TRY(make_map(&meh2, e_hi, M, dim, bkc, BN / 2));
-        HRAG_TRY(make_map(&mel2, e_lo, M, dim, bkc, BN / 2));
-        const int64_t work = (int64_t)ceil_div(Bq, 2 * BM) * p.num_n_tiles;
-        int g2 = (int)std::min<int64_t>(work, num_sms / 2) * 2;
-        if (const char* eg = getenv("HRAG_SIM_GRID")) g2 = std::max(2, std::min(g2, atoi(eg) & ~1));
-        if (fuse) k_sim_tc2<true><<<g2, TC_THREADS, SMEM_BYTES, stream>>>(mqh, mql, meh2, mel2, p);
-        else k_sim_tc2<false><<<g2, TC_THREADS, SMEM_BYTES, stream>>>(mqh, mql, meh2, mel2, p);
-        count_launch(1);
-        HRAG_CUDA(cudaGetLastError());
-        return 0;
-    }
+    const int grid = (int)std::min<int64_t>((int64_t)p.num_m_tiles * p.num_n_tiles, num_sms);
     if (n_seg == 4 && fuse) k_sim_tc<true, 1><<<grid, TC_THREADS, SMEM_BYTES, stream>>>(mqh, mql, meh, mel, p);
     else if (n_seg == 4) k_sim_tc<true, 0><<<grid, TC_THREADS, SMEM_BYTES, stream>>>(mqh, mql, meh, mel, p);
     else if (fuse) k_sim_tc<false, 1><<<grid, TC_THREADS, SMEM_BYTES, stream>>>(mqh, mql, meh, mel, p);

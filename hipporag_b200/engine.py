@@ -324,11 +324,9 @@ class Engine:
                                                 _ptr(scores), _ptr(found)))
         return ids, scores, found
 
-    def set_tuning(self, mixed_hint: int = -1, use_tma: int = -1, sorted_rows: int = -1, sweep_shape: int = -1,
-                   k5_debug: int = -1):
-        """Profiling switches: cache-policy variant of the fp16 sweep / TMA-gather sweep / by-length row
-        assignment / (gathers in flight, CTAs per SM)."""
-        _lib.check(self._lib.hrag_set_tuning(self._h, mixed_hint, use_tma, sorted_rows, sweep_shape, k5_debug))
+    def set_tuning(self, k5_debug: int = -1):
+        """Profiling switches of the fused multi-GPU exchange (hrag_set_tuning; -1 keeps the current value)."""
+        _lib.check(self._lib.hrag_set_tuning(self._h, k5_debug))
 
     def bench_sweep(self, batch: int, sweeps: int = 20, method: int = PPR_POWER) -> float:
         ms = C.c_float()

@@ -203,14 +203,10 @@ int hrag_knn_threshold(hrag_t* h, int which, int32_t B, const float* q, float mi
  * compact rhs of stage B (needs hrag_load_tables). */
 int hrag_bench_sweep(hrag_t* h, int32_t B, int32_t sweeps, int32_t method, float* ms_per_sweep);
 
-/* Kernel-variant switches for profiling (-1 keeps): mixed_hint = L2 cache-policy variant of the fp16 sweep
- * (0 none, 1 gathers evict_last + streams evict_first, 2 half of the gathers evict_last, 3 = 1 + gathers
- * bypass L1, 4 = gathers bypass L1 only, no L2 descriptors); use_tma = 1 routes the plain fp16 sweeps through the TMA-gather kernel (ppr_tma.cu);
- * sorted_rows = 0 disables the by-length assignment of a CTA's 64 rows to its warps; sweep_shape = gathers in
- * flight per lane / CTAs per SM of the fp16 sweep (0 = 4 / 6, 1 = 8 / 4, 2 = 6 / 5); k5_debug = timing probes of the
- * fused exchange (bit 0: no per-CTA system fence, bit 1: no peer stores -- results are INVALID with either; bit 2:
- * push the row blocks with LSU stores instead of TMA bulk copies -- valid, slower). */
-int hrag_set_tuning(hrag_t* h, int mixed_hint, int use_tma, int sorted_rows, int sweep_shape, int k5_debug);
+/* Profiling switches (-1 keeps): k5_debug = timing probes of the fused exchange (bit 0: no per-CTA system fence,
+ * bit 1: no peer stores -- results are INVALID with either; bit 2: push the row blocks with LSU stores instead of
+ * TMA bulk copies -- valid, slower). */
+int hrag_set_tuning(hrag_t* h, int k5_debug);
 
 /* The CUDA stream (cudaStream_t) every kernel and copy of this handle is issued on, so a
  * caller can bracket calls with its own CUDA events. */

@@ -45,6 +45,17 @@ def test_product_never_imports_the_oracle():
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), f"{f} imports oracle/"
 
 
+def test_native_code_reads_only_the_exchange_switches():
+    """Kernel variants are chosen by the code, not by environment switches: the only variables the native
+    library reads are the two of the multi-GPU exchange."""
+    csrc = os.path.join(ROOT, "hipporag_b200", "csrc")
+    names = set()
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh", ".h")):
+            names |= set(re.findall(r'getenv\(\s*"([^"]+)"', open(os.path.join(csrc, f)).read()))
+    assert names == {"HRAG_K5_MODE", "HRAG_MIXED_PERSIST"}
+
+
 def test_transition_csr_matches_oracle_restating():
     from hipporag_b200.engine import build_transition_csr
     from oracle import ppr

@@ -186,23 +186,6 @@ def test_ppr_sweep_counts_follow_damping(hb, damping, batch):
         assert np.max(np.abs(got2 - want) / scale) < RTOL
 
 
-def test_tma_gather_sweep_equals_ldg_sweep(hb):
-    """K1t (TMA gather4 into a shared-memory ring) computes the same sweep as k_sweep_h, bit for bit."""
-    from hipporag_b200 import synth
-    kg = synth.make_kg(30_000, 300_000, seed=6)
-    rng = np.random.default_rng(1)
-    R = np.zeros((33, kg.n_nodes), dtype=np.float32)
-    R[:, kg.passage_vid] = 0.05 * rng.random((33, kg.n_pass), dtype=np.float32)
-    for b in range(33):
-        R[b, rng.integers(0, kg.n_ent, 5)] = rng.random(5, dtype=np.float32)
-    e = _engine_for_graph(hb, kg.n_nodes, kg.edge_src, kg.edge_dst, kg.edge_w)
-    a = e.ppr(R)
-    e.set_tuning(use_tma=1)
-    b = e.ppr(R)
-    e.set_tuning(use_tma=0)
-    np.testing.assert_array_equal(a, b)
-
-
 def test_retrieve_musique1k_mixed_precision(hb, golden, c1):
     g = golden
     c1.engine.set_options(ppr_precision=hb.PPR_MIXED)
@@ -280,27 +263,6 @@ def test_similarity_modes_vs_float64(hb, dim, rows, bq):
             for b in range(0, bq, 17):
                 assert_topk_matches(idx[b], score[b], retrieve.min_max_normalize(want[b]), 5, what=f"mode {mode} q{b}")
     assert idx[0, 0] == 3
-
-
-def test_two_cta_gemm_variant_in_a_subprocess():
-    """The cta_group::2 kernel (HRAG_SIM_2CTA=1, read once per process) must give the same answers."""
-    import subprocess, sys, os
-    code = (
-        "import numpy as np, hipporag_b200 as hb\n"
-        "from hipporag_b200 import synth\n"
-        "E = synth.unit_rows(3000, 768, seed=1); Q = synth.unit_rows(300, 768, seed=2); Q[0] = E[3]\n"
-        "e = hb.Engine(0); e.load_embeddings(E, synth.unit_rows(8, 768, seed=9))\n"
-        "i1, s1, _ = e.stage_a(Q, 5)\n"
-        "e.debug_keep_scores(True); i2, s2, _ = e.stage_a(Q, 5); got = e.debug_scores(0)\n"
-        "want = Q.astype(np.float64) @ E.astype(np.float64).T\n"
-        "assert np.array_equal(i1, i2) and np.array_equal(s1, s2)\n"
-        "assert np.max(np.abs(got - want)) < 8e-6, np.max(np.abs(got - want))\n"
-        "assert i1[0, 0] == 3\n"
-        "print('2cta ok')\n")
-    env = dict(os.environ, HRAG_SIM_2CTA="1")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0 and "2cta ok" in out.stdout, out.stdout + out.stderr
 
 
 def test_knn_matches_exact_cosine_topk(hb):

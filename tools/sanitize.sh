@@ -26,13 +26,10 @@ R = np.random.default_rng(0).random((3, kg.n_nodes), dtype=np.float32)
 r.engine.ppr(R)
 r.engine.ppr(np.random.default_rng(1).random((20, kg.n_nodes), dtype=np.float32), damping=0.85)
 r.engine.similarity(1, qp[:3])
-# round-2 kernels: linking_top_k > 8 (radix select path + 64 seed slots), threshold KNN epilogue, TMA-gather sweep
+# round-2 kernels: linking_top_k > 8 (radix select path + 64 seed slots), threshold KNN epilogue
 idx, score, nv = r.engine.stage_a(qf, 10)
 r.engine.stage_b(qp, idx, score, link_top_k=10, topk=50)
 r.engine.knn_threshold(0, fe[:200], 0.3, 64)
-r.engine.set_tuning(use_tma=1)
-r.engine.ppr(np.random.default_rng(2).random((33, kg.n_nodes), dtype=np.float32))
-r.engine.set_tuning(use_tma=0)
 print("driver ok", ids.shape)
 PY
 compute-sanitizer --tool $TOOL --error-exitcode 7 python /tmp/hrag_sanitize_driver.py 2>&1 | tail -15
